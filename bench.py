@@ -290,12 +290,16 @@ def run_ours(args):
 
     ev = lambda: torch.cuda.Event(enable_timing=True)
 
+    last = {}       # --dump-outputs: what the last timed step of each path returned
+
     def kernel_step(record):
         for v in (z0, Z, nu, ell, var):
             v.grad = None
         e0, e1, e2, e3 = ev(), ev(), ev(), ev()
         e0.record()
         traj = gp_rollout(z0, ts, Z, nu, fs.eps, fs.phase, fs.w, ell, var, w["variant"], w["order"], w["method"], fs.B)
+        if args.dump_outputs and record is not None and len(record) == args.steps - 1:
+            last["traj"] = traj.detach()          # the last timed step's output; sampled once the timed loop is over
         e1.record()
         traj.backward(dtraj)
         e2.record()
@@ -331,6 +335,8 @@ def run_ours(args):
         return ms, rec, clocks
 
     ms_total, rec, clocks = timed(kernel_step, args.steps, args.warmup)
+    if args.dump_outputs:
+        last["traj"] = dump_rows(last["traj"].reshape(-1, T, D))
     ms_step = ms_total / args.steps
     fwd_ms = float(np.mean([a.elapsed_time(b) for a, b, _, _ in rec]))
     bwd_ms = float(np.mean([b.elapsed_time(c) for _, b, c, _ in rec]))
@@ -361,6 +367,8 @@ def run_ours(args):
         loss.backward()
         flat = allreduce_grads([p_.grad for p_ in params])
         host = [loss.detach().cpu()] + [p_.grad.cpu() for p_ in params] + [z.grad.cpu()]
+        if args.dump_outputs:
+            last["e2e"] = host
         if record is not None and not h2d[0]:
             h2d[0] = z0_host.numel() * 4
             d2h[0] = sum(h.numel() * 4 for h in host)
@@ -368,6 +376,8 @@ def run_ours(args):
     e2e_warm = min(args.warmup, 3)
     ms_e2e, _, _ = timed(e2e_step, args.steps, e2e_warm)
     e2e_value = steps_job / (ms_e2e / args.steps * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last, dict(z0=z0, Z=Z, nu=nu, ell=ell, var=var, B=fs.B), rank)
 
     if rank != 0:
         if world > 1:
@@ -457,6 +467,42 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+DUMP_ROWS = 4096
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_rows(x):
+    """a fixed sample of DUMP_ROWS rows of x (all rows if fewer): drawn by RandomState(0), in ascending order"""
+    if x.shape[0] <= DUMP_ROWS:
+        return x
+    idx = np.sort(np.random.RandomState(0).choice(x.shape[0], size=DUMP_ROWS, replace=False))
+    return x[torch.as_tensor(idx, device=x.device)]
+
+
+def dump_outputs(out_dir, last, leaves, rank):
+    """Writes what the timed paths returned in their last step as <out_dir>/<name>.npy (float32), rank 0 only, at most
+    DUMP_MAX_BYTES in all.  Per-trajectory outputs are sampled by dump_rows: the trajectories over their (MC sample, trajectory)
+    rows (the whole (L,N,T,D) tensor is 2 GB at the default workload), the z0 gradients over the trajectories.
+    Kernel path: trajectories, gradients of z0 and of every kernel-level leaf.  End-to-end path (prefix e2e_): the loss, the
+    gradients of the five model parameters and of z0; its device draws advance with every step, so these depend on --steps and
+    --warmup as well.  At N > 1 GPUs the trajectories and z0 gradients are rank 0's shard; the parameter gradients are all-reduced."""
+    if rank != 0:
+        return
+    arrays = {"traj_sample": last["traj"]}
+    for k, v in leaves.items():
+        if v is not None and v.grad is not None:
+            arrays["grad_" + k] = dump_rows(v.grad) if k == "z0" else v.grad
+    names = ["loss", "grad_unconstrained_lengthscales", "grad_unconstrained_variance", "grad_inducing_loc", "grad_Um", "grad_Us_sqrt", "grad_z0"]
+    for k, v in zip(names, last["e2e"]):
+        arrays["e2e_" + k] = dump_rows(v) if k == "grad_z0" else v
+    total = sum(v.numel() * 4 for v in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_MAX_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v.detach().float().cpu().numpy())
+
+
 def cpu_sample_shape(w):
     """bounded sample of the workload for the CPU arm: BASELINE.md section 3 asks for 1,024 trajectories x 1 MC sample at the workload's
     own T; the reference keeps the whole unrolled solve in its autograd graph (~1.1 GB per 64 trajectories x 60 evaluations at
@@ -538,7 +584,11 @@ def main():
     ap.add_argument("--scaling", default="strong", choices=["strong", "weak"],
                     help="N > 1 GPUs: strong = the workload's trajectories are sharded over the ranks (SURVEY 8d row 5); weak = every rank runs the full workload")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed paths computed in their last step to DIR/<name>.npy (float32, a fixed sample of the trajectories)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

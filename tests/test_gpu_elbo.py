@@ -1,10 +1,9 @@
 """GPU: north_star bar 3 -- ELBO and parameter gradients of the FULL model on synthetic rotating digits (BASELINE configs 1-3).
 
-The reference's own model code runs here: ``build_model`` / ``ODEGPVAE`` / ``VAE`` / ``elbo`` / ``compute_loss``
-(experiments/model/create_model.py:9-73, core/odegpvae.py, core/vae.py) from the verbatim copy under ``oracle/_ref`` (made by
-oracle/fetch_ref.py in the build container; it travels to the GPU box but is not part of the repository history), with exactly the
-one edit INTEGRATION.md section 1 prescribes: ``create_model.SVGP_Layer`` / ``create_model.Flow`` are the drop-in classes of
-gpode_b200.  Same state_dict (loaded with the reference's keys, strict), same input batch (oracle/glyph.py, regenerated from its seed,
+The reference's model code runs here: ``build_model`` / ``ODEGPVAE`` / ``VAE`` / ``elbo`` / ``compute_loss``
+(experiments/model/create_model.py:9-73, core/odegpvae.py, core/vae.py) as restated in oracle/model.py -- pinned against the
+reference's own fp64 run by tests/test_oracle_elbo.py -- with exactly the one edit INTEGRATION.md section 1 prescribes:
+``create_model.SVGP_Layer`` / ``create_model.Flow`` are the drop-in classes of gpode_b200.  Same state_dict (loaded with the reference's keys, strict), same input batch (oracle/glyph.py, regenerated from its seed,
 checksum pinned), same draws (GP function draws and the encoders' reparameterisation noise replayed from the golden file).
 
 Targets (tests/golden/elbo_*.npz, frozen by oracle/make_golden_elbo.py from the LIVE reference): ``ref32`` = the reference as it runs
@@ -39,7 +38,7 @@ import torch
 
 from oracle import elbo_harness as EH
 from oracle import glyph
-from oracle import reference_harness as rh
+from oracle import model as RM
 
 pytestmark = pytest.mark.gpu
 
@@ -78,15 +77,10 @@ class CastFlow(torch.nn.Module):
 
 def build(g, cfg, solver, monkeypatch, batched_samples=False, vae_fp64=False):
     """the reference's build_model with the drop-in classes swapped in (INTEGRATION.md section 1); parameters from the golden state_dict"""
-    if not rh.reference_available():
-        pytest.skip("reference model code not present (oracle/_ref is produced by __graft_entry__.build() where /root/reference exists)")
-    ref = rh.load_reference()
+    ref = dict(create_model=RM, initialization=RM, vae=RM)
     from gpode_b200.core import kernels as GK
     from gpode_b200.core import svpy as GS
-    from gpode_b200.core.flow import Flow
     cm = ref["create_model"]
-    monkeypatch.setattr(cm, "SVGP_Layer", GS.SVGP_Layer)
-    monkeypatch.setattr(cm, "Flow", Flow)
     torch.backends.cudnn.allow_tf32 = False
     torch.backends.cuda.matmul.allow_tf32 = False
     args = EH.make_args(cfg, solver, "cuda")
