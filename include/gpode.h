@@ -35,7 +35,7 @@ enum {
   GPODE_OK = 0,
   GPODE_E_NULL = -1,        /* a required pointer is NULL */
   GPODE_E_SHAPE = -2,       /* a size is non-positive or inconsistent (e.g. DF with D_in != D_out) */
-  GPODE_E_UNSUPPORTED = -3, /* shape outside the compiled range (D_in > 16, DF D > 8, parameter tile > 227 KB ...) */
+  GPODE_E_UNSUPPORTED = -3, /* shape outside the compiled range (D_in > 16, DF D > 8, L > 65535, parameter tile > 227 KB ...) */
   GPODE_E_WORKSPACE = -4,   /* workspace / save buffer too small or misaligned */
   GPODE_E_ENUM = -5         /* unknown variant / method / order */
 };
@@ -57,7 +57,7 @@ enum {
  */
 typedef struct GpodeProblem {
   int32_t variant;
-  int32_t L;      /* MC samples (independent function samples) */
+  int32_t L;      /* MC samples (independent function samples), at most 65535: the launches put L on grid y / z */
   int32_t N;      /* states (trajectories) per sample */
   int32_t D_in;   /* GP input dim = ODE state dim (order 1: q, order 2: 2q) */
   int32_t D_out;  /* GP output dim */

@@ -31,6 +31,25 @@ def test_library_exports_every_declared_symbol():
     assert L.gpode_field_fwd(ctypes.byref(p), None, None, None, None, 0, None) < 0
 
 
+
+@pytest.mark.parametrize("variant", ["rbf_dimwise", "df"])
+def test_sample_count_limit(variant):
+    """every sweep, pack and parameter-gradient launch puts the sample index L on grid y or z (at most 65,535): a larger L is refused
+    with GPODE_E_UNSUPPORTED by the argument check, before any CUDA call, instead of failing at launch"""
+    from gpode_b200 import _lib
+    L = _lib.load()
+    dummy = ctypes.c_void_p(256)          # never dereferenced: the shape check comes first
+    p = _lib.GpodeProblem()
+    p.variant, p.N, p.D_in, p.D_out, p.M, p.S = _lib.VARIANTS[variant], 2, 4, 4, 8, 8
+    p.Z = p.ell = p.var = p.eps = p.phase = p.w = p.nu = p.B = dummy
+    for Lm, ok in ((65535, True), (65536, False), (1 << 20, False)):
+        p.L = Lm
+        assert (L.gpode_workspace_bytes(ctypes.byref(p), 3, _lib.RK4) > 0) == ok, Lm
+        assert (L.gpode_rollout_save_floats(ctypes.byref(p), 3, _lib.RK4) > 0) == ok, Lm
+        if not ok:
+            assert L.gpode_field_fwd(ctypes.byref(p), dummy, dummy, dummy, dummy, 0, None) == -3      # GPODE_E_UNSUPPORTED
+    assert b"L <= 65535" in L.gpode_error_string(-3)
+
 def test_forward_kernel_selection(monkeypatch):
     """which forward kernel family a problem gets depends on shapes only (plus GpodeProblem.flags): no CUDA call involved, and no
     environment variable is read"""

@@ -25,6 +25,7 @@ int check_problem(const GpodeProblem* p) {
   if (!p->Z || !p->ell || !p->var || !p->eps || !p->phase || !p->w || !p->nu) return GPODE_E_NULL;
   if (p->D_in > kMaxD || p->D_out > kMaxD || p->M > 512) return GPODE_E_UNSUPPORTED;
   if (static_cast<long>(p->L) * p->N > (1L << 30)) return GPODE_E_UNSUPPORTED;
+  if (p->L > kMaxSamples) return GPODE_E_UNSUPPORTED;   // every sweep, pack and parameter-gradient launch puts L on grid y or z
   if (p->variant == GPODE_DF) {
     if (p->D_in != p->D_out) return GPODE_E_SHAPE;
     if (!p->B) return GPODE_E_NULL;
@@ -276,7 +277,7 @@ const char* gpode_error_string(int code) {
     case GPODE_OK: return "ok";
     case GPODE_E_NULL: return "a required pointer is NULL";
     case GPODE_E_SHAPE: return "invalid or inconsistent shape";
-    case GPODE_E_UNSUPPORTED: return "shape outside the compiled range (D_in/D_out <= 16, DF D <= 8, M <= 512, parameter tile <= 227 KB)";
+    case GPODE_E_UNSUPPORTED: return "shape outside the compiled range (D_in/D_out <= 16, DF D <= 8, M <= 512, L <= 65535, L*N <= 2^30, parameter tile <= 227 KB)";
     case GPODE_E_WORKSPACE: return "workspace too small or not 256-byte aligned";
     case GPODE_E_ENUM: return "unknown variant / method / order";
     default: return code > 0 ? cudaGetErrorString(static_cast<cudaError_t>(code)) : "unknown error";

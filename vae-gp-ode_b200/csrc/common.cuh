@@ -20,6 +20,7 @@ namespace gpode {
 constexpr float kLog2e = 1.4426950408889634f;
 constexpr float kLn2 = 0.6931471805599453f;
 constexpr int kMaxD = 16;          // largest GP input dimension compiled
+constexpr int kMaxSamples = 65535;  // largest L: the launches put the sample index on grid y or z
 constexpr int kMaxStages = 4;
 constexpr int kSmemLimit = 227 * 1024;
 
